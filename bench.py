@@ -2,7 +2,7 @@
 """bench.py -- compress MB/s at -9 (BASELINE.json metric), one JSON line on rank 0.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload text|random|period1000|aab|runs|mixed]
-                  [--mb 1000] [--level 9] [--engines-per-gpu 2] [--no-c4] [--sweep]
+                  [--mb 1000] [--level 9] [--engines-per-gpu 2] [--no-c4] [--sweep] [--dump-outputs DIR]
 
 A "step" is one pass of the whole compression path (RLE1+CRC -> BWT -> MTF/RLE2 -> Huffman -> stream)
 over one synthetic input of --mb MB per GPU (default: the 1 GB Zipf text of SURVEY.md 8(d) C2, BASELINE.json
@@ -15,6 +15,9 @@ configs[1]); at N GPUs the input is ONE stream of N x --mb MB, sharded by block 
   cpu_baseline  the reference's own CPU path (oracle/_ref) on a bounded sample, single thread
   parity_checked_bytes   bytes of the timed output compared equal with the reference's stream of a prefix
   c4     secondary line: SURVEY 8(d) C4, 16 GB mixed, strong-scaled over the N GPUs
+
+--dump-outputs DIR writes what the last timed step handed its caller (see dump_outputs) as .npy files, so that two
+builds run with the same arguments, hence on the same seeded input, can be compared output for output.
 
 The work is driven through the C API of libbz2_b200.so by ONE process: under torchrun (N > 1) rank 0 drives all N
 GPUs (csrc/multi.cu: windows round-robin over the engines, two host integers chain them, no collective on the data
@@ -323,6 +326,24 @@ class Samplers:
         return merge_clocks([x.summary() for x in self.s]) if len(self.s) > 1 else self.s[0].summary()
 
 
+DUMP_SAMPLE = 4 << 20          # stream bytes kept by --dump-outputs: 16 MB of float32 values + 32 MB of float64 positions
+
+
+def dump_outputs(path, stream, st):
+    """The .bz2 stream of the last timed step and the counts the C API returned with it.
+      stream_bytes.npy  float32, the stream's bytes at the positions in stream_index.npy (all of them up to DUMP_SAMPLE
+                        bytes, else a sample drawn with a fixed seed)
+      stream_index.npy  float64, those positions, ascending
+      stream_stats.npy  float64 [in_bytes, out_bytes, n_blocks, combined_crc, sum_nblock, sum_nmtf, n_power_blocks, out_bits]"""
+    os.makedirs(path, exist_ok=True)
+    n = stream.size
+    idx = np.arange(n) if n <= DUMP_SAMPLE else np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))
+    np.save(os.path.join(path, "stream_bytes.npy"), stream[idx].astype(np.float32))
+    np.save(os.path.join(path, "stream_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(path, "stream_stats.npy"), np.array([st.in_bytes, st.out_bytes, st.n_blocks, st.combined_crc, st.sum_nblock,
+                                                              st.sum_nmtf, st.n_power_blocks, st.out_bits], np.float64))
+
+
 def equal_prefix(a, b):
     n = min(a.size, b.size)
     ne = np.nonzero(a[:n] != b[:n])[0]
@@ -407,7 +428,10 @@ def main():
     ap.add_argument("--c4-gb", type=float, default=16.0)
     ap.add_argument("--sweep", action="store_true", help="C5: -1..-9 on --sweep-gb GB of text, outputs decoded by oracle/_ref/bzip2_ref")
     ap.add_argument("--sweep-gb", type=float, default=4.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output stream and counts as .npy files to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -526,6 +550,8 @@ def main():
     out_len = job.out_len
     launches = int(st.kernel_launches) * args.steps
     out_resident = job.h_out[:out_len].numpy().copy()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out_resident, st)
     job.drop_resident()
 
     e2e = None
