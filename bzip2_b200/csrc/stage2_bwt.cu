@@ -131,6 +131,7 @@ constexpr int KG_MAXK = 24;
 constexpr u32 KG_TAB_LOG2 = 13;             // per-tile k-gram table of the count pass: 8192 slots for 4096 positions
 constexpr u32 KG_TAB = 1u << KG_TAB_LOG2;
 constexpr u32 KG_AGG_MAX_ALPHA = 128;       // aggregate per tile for alphabets up to this size (byte-wide data has few repeats per tile)
+constexpr u32 KG_AGG_MAX_BINS = 1u << 19;   // ... and bin counts below this: a slot word holds key + 1 in 19 bits above a 13-bit count
 
 enum { KG_HISTOFF = 3, KG_PLACE = 4 };
 
@@ -207,7 +208,7 @@ __global__ void __launch_bounds__(KG_THREADS) k_kgram(S2Params p)
       sc[s] = cmap[T[gi]];
    }
    __syncthreads();
-   if (AGG && base <= p.kg_agg_alpha) {
+   if (AGG && base <= p.kg_agg_alpha && p.nbins[b] < KG_AGG_MAX_BINS) {
       // Count pass with per-tile aggregation.  10^8 returning global atomics run at the L2's atomic rate (81 G/s, round 1:
       // 1.25 ms per window) -- but on text only ~22 % of the k-grams of a 4096-position tile are distinct.  The tile first
       // counts its k-grams in a shared-memory hash table (slot word = key+1 << 13 | count; an element's arrival index

@@ -216,9 +216,11 @@ static int32_t hb_pop(hb_t* h)
    hb_down(h, 1);
    return top;
 }
-void orc_make_code_lengths(int32_t* len, const int32_t* freq, int32_t alpha, int32_t max_len)
+/* returns how many times the weights were halved to meet max_len */
+static int32_t make_code_lengths(int32_t* len, const int32_t* freq, int32_t alpha, int32_t max_len)
 {
    hb_t h;
+   int32_t halvings = 0;
    for (int32_t i = 0; i < alpha; i++) h.w[i + 1] = (freq[i] == 0 ? 1 : freq[i]) << 8;
    for (;;) {
       int32_t nnodes = alpha;
@@ -242,8 +244,14 @@ void orc_make_code_lengths(int32_t* len, const int32_t* freq, int32_t alpha, int
          if (d > max_len) too_long = 1;
       }
       if (!too_long) break;
+      halvings++;
       for (int32_t i = 1; i <= alpha; i++) h.w[i] = (1 + (h.w[i] >> 8) / 2) << 8;
    }
+   return halvings;
+}
+void orc_make_code_lengths(int32_t* len, const int32_t* freq, int32_t alpha, int32_t max_len)
+{
+   (void)make_code_lengths(len, freq, alpha, max_len);
 }
 void orc_assign_codes(int32_t* code, const int32_t* len, int32_t min_len, int32_t max_len, int32_t alpha)
 {
@@ -255,21 +263,24 @@ void orc_assign_codes(int32_t* code, const int32_t* len, int32_t min_len, int32_
 }
 
 /* ------------------------------------------------------------ bit writer -- */
-/* compress.c:37-86: MSB-first.  `out` must be zero beyond *bitpos. */
+/* compress.c:37-86: MSB-first.  `out` must be zero beyond *bitpos; out == NULL only counts the bits. */
 static void put_bits(uint8_t* out, uint64_t* bitpos, int nb, uint32_t v)
 {
    uint64_t p = *bitpos;
+   if (!out) { *bitpos = p + (uint64_t)nb; return; }
    for (int k = nb - 1; k >= 0; k--, p++)
       if ((v >> k) & 1) out[p >> 3] |= (uint8_t)(0x80u >> (p & 7));
    *bitpos = p;
 }
 
 /* ------------------------------------------------------- sendMTFValues -- */
-void orc_send_mtf(const uint16_t* mtfv, int32_t n_mtf, const uint8_t* in_use,
-                  const int32_t* mtf_freq, uint8_t* out, uint64_t* bitpos)
+/* The body of orc_send_mtf and orc_send_mtf_tables: selectors go to sel (nsel entries), the final code lengths
+ * to len, the halving count of every (pass, table) to halvings (or nowhere if NULL).  Returns nGroups. */
+static int send_mtf(const uint16_t* mtfv, int32_t n_mtf, const uint8_t* in_use, const int32_t* mtf_freq,
+                    uint8_t* out, uint64_t* bitpos, uint8_t* sel, int32_t len[6][258], int32_t halvings[4][6])
 {
    static const int NG_MAX = 6, GS = 50;
-   int32_t len[6][258], code[6][258], fr[6][258];
+   int32_t code[6][258], fr[6][258];
    int32_t n_in_use = 0;
    for (int c = 0; c < 256; c++) n_in_use += in_use[c] ? 1 : 0;
    const int32_t alpha = n_in_use + 2;
@@ -288,7 +299,6 @@ void orc_send_mtf(const uint16_t* mtfv, int32_t n_mtf, const uint8_t* in_use,
       }
    }
    int32_t nsel = (n_mtf + GS - 1) / GS;
-   uint8_t* sel = malloc((size_t)nsel + 1);
    /* refinement passes, compress.c:324-561 */
    for (int it = 0; it < 4; it++) {
       memset(fr, 0, sizeof fr);
@@ -301,7 +311,10 @@ void orc_send_mtf(const uint16_t* mtfv, int32_t n_mtf, const uint8_t* in_use,
          sel[g] = (uint8_t)bt;
          for (int32_t i = lo; i < hi; i++) fr[bt][mtfv[i]]++;
       }
-      for (int t = 0; t < ng; t++) orc_make_code_lengths(len[t], fr[t], alpha, 17);
+      for (int t = 0; t < ng; t++) {
+         const int32_t h = make_code_lengths(len[t], fr[t], alpha, 17);
+         if (halvings) halvings[it][t] = h;
+      }
    }
    for (int t = 0; t < ng; t++) {
       int32_t mn = 32, mx = 0;
@@ -346,7 +359,27 @@ void orc_send_mtf(const uint16_t* mtfv, int32_t n_mtf, const uint8_t* in_use,
       int t = sel[i / GS];
       put_bits(out, bitpos, len[t][mtfv[i]], (uint32_t)code[t][mtfv[i]]);
    }
+   return ng;
+}
+
+void orc_send_mtf(const uint16_t* mtfv, int32_t n_mtf, const uint8_t* in_use,
+                  const int32_t* mtf_freq, uint8_t* out, uint64_t* bitpos)
+{
+   int32_t len[6][258];
+   uint8_t* sel = malloc((size_t)(n_mtf + 49) / 50 + 1);
+   (void)send_mtf(mtfv, n_mtf, in_use, mtf_freq, out, bitpos, sel, len, NULL);
    free(sel);
+}
+
+int32_t orc_send_mtf_tables(const uint16_t* mtfv, int32_t n_mtf, const uint8_t* in_use, const int32_t* mtf_freq,
+                            uint8_t* sel, int32_t len[6][258], int32_t halvings[4][6], uint64_t* coded_bits)
+{
+   uint64_t bits = 0;
+   memset(len, 0, sizeof(int32_t) * 6 * 258);
+   memset(halvings, 0, sizeof(int32_t) * 4 * 6);
+   const int ng = send_mtf(mtfv, n_mtf, in_use, mtf_freq, NULL, &bits, sel, len, halvings);
+   *coded_bits = bits;
+   return ng;
 }
 
 /* ---------------------------------------------------------- whole stream -- */

@@ -71,6 +71,13 @@ void orc_assign_codes(int32_t* code, const int32_t* len, int32_t min_len, int32_
 void orc_send_mtf(const uint16_t* mtfv, int32_t n_mtf, const uint8_t* in_use,
                   const int32_t* mtf_freq, uint8_t* out, uint64_t* bitpos);
 
+/* The same computation, returning what it decided instead of the bits: nGroups (the return value), the final
+ * selector of every 50-symbol group (sel: (n_mtf + 49) / 50 entries), the final code lengths of every table
+ * (len; tables >= nGroups and symbols >= nInUse + 2 are 0), how many times each of the 4 passes halved each
+ * table's weights to meet the 17-bit limit, and the bit length of the coded section (symbol map onwards). */
+int32_t orc_send_mtf_tables(const uint16_t* mtfv, int32_t n_mtf, const uint8_t* in_use, const int32_t* mtf_freq,
+                            uint8_t* sel, int32_t len[6][258], int32_t halvings[4][6], uint64_t* coded_bits);
+
 /* Whole stream (compress.c:822-881 framing).  force_orig_ptr: optional array
  * (one per block, or NULL) overriding origPtr where >= 0 (used to inject the
  * reference's tie-break on exact-power blocks). Returns bytes written or <0. */

@@ -53,6 +53,9 @@ def oracle():
     lib.orc_make_code_lengths.argtypes = [C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int32, C.c_int32]
     lib.orc_send_mtf.restype = None
     lib.orc_send_mtf.argtypes = [C.POINTER(C.c_uint16), C.c_int32, u8p, C.POINTER(C.c_int32), u8p, C.POINTER(C.c_uint64)]
+    lib.orc_send_mtf_tables.restype = C.c_int32
+    lib.orc_send_mtf_tables.argtypes = [C.POINTER(C.c_uint16), C.c_int32, u8p, C.POINTER(C.c_int32), u8p,
+                                        C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_uint64)]
     lib.orc_compress.restype = C.c_int64
     lib.orc_compress.argtypes = [u8p, C.c_uint64, C.c_int, C.c_int, C.POINTER(C.c_int32), u8p, C.c_uint64]
     lib.gen_text.restype = C.c_uint64
@@ -151,7 +154,7 @@ def ref_bwt(block):
 
 def orc_split(data, level=9, tail_merge=1):
     a = as_u8(data)
-    maxb = a.size // (100000 * level - 30) + 3
+    maxb = (a.size + a.size // 4) // (100000 * level - 30) + 3       # RLE1 turns a run of four into five bytes
     blocks = (OrcBlock * maxb)()
     nb = oracle().orc_rle1_split(_buf(a), a.size, level, tail_merge, blocks, maxb)
     assert 0 <= nb <= maxb
@@ -190,6 +193,21 @@ def orc_mtf(bwt, inuse):
     return mtfv[:n].copy(), freq, nu.value
 
 
+def orc_send_mtf_tables(mtfv, freq, inuse):
+    """Stage 4's decisions for one block: (nGroups, selectors, code lengths [6][258], halvings [4 passes][6 tables],
+    bits of the coded section from the symbol map on)."""
+    m = np.ascontiguousarray(mtfv, dtype=np.uint16)
+    f = np.ascontiguousarray(freq, dtype=np.int32)
+    iu = as_u8(inuse)
+    sel = np.zeros((m.size + 49) // 50 + 1, np.uint8)
+    lens = np.zeros((6, 258), np.int32)
+    halv = np.zeros((4, 6), np.int32)
+    bits = C.c_uint64(0)
+    ng = oracle().orc_send_mtf_tables(_p(m, C.c_uint16), m.size, _p(iu), _p(f, C.c_int32), _p(sel), _p(lens, C.c_int32),
+                                      _p(halv, C.c_int32), C.byref(bits))
+    return ng, sel[: (m.size + 49) // 50].copy(), lens, halv, bits.value
+
+
 def orc_compress(data, level=9, tail_merge=1, force_orig_ptr=None):
     a = as_u8(data)
     cap = int(a.size * 1.3) + 100000
@@ -201,6 +219,31 @@ def orc_compress(data, level=9, tail_merge=1, force_orig_ptr=None):
     n = oracle().orc_compress(_buf(a), a.size, level, tail_merge, fp, _p(out), cap)
     assert n > 0, n
     return out[:n].tobytes()
+
+
+# ----------------------------------------------------------------------------- stage 2 parameters
+def hist_stride(level, hist_log2=18):
+    """k-gram bins reserved per block (engine_new, csrc/engine.cu; BZ2_B200_HIST_LOG2 = hist_log2)"""
+    nmax = 100000 * level - 19
+    s = 1 << 16
+    while s < (1 << hist_log2) and s < nmax // 4:
+        s <<= 1
+    if hist_log2 > 18 and s < nmax * 2:
+        s = 1 << hist_log2
+    return s
+
+
+def codemap(ninuse, stride, maxk=24):
+    """k_codemap (csrc/stage2_bwt.cu): (k, nbins, bits per symbol, m) of a block with `ninuse` symbols.  The k-gram
+    sort starts at depth k with ninuse^k buckets; a text key holds the next m symbols in m * bits <= 51 bits."""
+    k, bins = 1, max(ninuse, 1)
+    while ninuse > 1 and k < maxk and bins * ninuse <= stride:
+        bins *= ninuse
+        k += 1
+    bits = 1
+    while (1 << bits) < ninuse:
+        bits += 1
+    return k, bins, bits, min(51 // bits, 48)
 
 
 # ----------------------------------------------------------------------------- generators
