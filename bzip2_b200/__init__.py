@@ -6,5 +6,5 @@ libbz2-compatible C front end).  This package is only a thin ctypes loader used 
 every call fails loudly if the library is missing or no CUDA device is usable.
 """
 from .binding import (  # noqa: F401
-    LIB_PATH, Bz2B200Error, Engine, Multi, Stats, bzlib, compress, build_library, load,
+    LIB_PATH, Bz2B200Error, Engine, Multi, Stats, bzlib, compress, compress_bound, build_library, load,
 )

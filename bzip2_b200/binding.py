@@ -47,6 +47,7 @@ EXPORTS = [
     "bz2b200_stream_feed", "bz2b200_debug_keep", "bz2b200_debug_fetch",
     "bz2b200_scan_create", "bz2b200_scan_rescan", "bz2b200_scan_boundary", "bz2b200_scan_destroy", "bz2b200_concat_bits",
     "bz2b200_multi_create", "bz2b200_multi_destroy", "bz2b200_multi_engines", "bz2b200_multi_compress",
+    "bz2b200_compress_bound", "bz2b200_engine_create_batch", "bz2b200_compress_batch_host", "bz2b200_compress_batch_device",
     # include/bzlib.h
     "BZ2_bzCompressInit", "BZ2_bzCompress", "BZ2_bzCompressEnd", "BZ2_bzBuffToBuffCompress",
     "BZ2_bzWriteOpen", "BZ2_bzWrite", "BZ2_bzWriteClose", "BZ2_bzWriteClose64", "BZ2_bzlibVersion",
@@ -133,6 +134,14 @@ def load():
     lib.bz2b200_multi_compress.restype = C.c_int
     lib.bz2b200_multi_compress.argtypes = [vp, vp, C.POINTER(vp), sz, vp, C.POINTER(sz), C.c_uint, C.POINTER(Stats)]
     lib.bz2b200_pool_clear.restype = None
+    lib.bz2b200_compress_bound.restype = sz
+    lib.bz2b200_compress_bound.argtypes = [C.c_int, sz]
+    lib.bz2b200_engine_create_batch.restype = C.c_int
+    lib.bz2b200_engine_create_batch.argtypes = [C.POINTER(vp), C.c_int, C.c_int, sz, sz]
+    u64p, u32p = C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)
+    for name in ("bz2b200_compress_batch_host", "bz2b200_compress_batch_device"):
+        getattr(lib, name).restype = C.c_int
+        getattr(lib, name).argtypes = [vp, vp, u64p, sz, vp, sz, u64p, u32p, C.c_uint, C.POINTER(Stats)]
     return lib
 
 
@@ -145,14 +154,28 @@ def _ptr(a):
     return a.ctypes.data if a.size else None
 
 
+def _u64p(a):
+    return a.ctypes.data_as(C.POINTER(C.c_uint64)) if a is not None else None
+
+
+def compress_bound(level, n):
+    """Worst-case size of one stream of n input bytes (the reference's BuffToBuff bound, 1% + 600 bytes)."""
+    return load().bz2b200_compress_bound(level, n)
+
+
 class Engine:
     """One GPU compression engine (bz2b200_engine_*)."""
 
-    def __init__(self, level=9, device=0, window_bytes=0):
+    def __init__(self, level=9, device=0, window_bytes=0, max_items=0):
+        """max_items != 0: an engine whose windows hold up to max_items inputs of a batch call (engine_create_batch)."""
         self.lib = load()
         self.h = C.c_void_p()
         self.level = level
-        _check(self.lib.bz2b200_engine_create(C.byref(self.h), device, level, window_bytes), "engine_create")
+        if max_items:
+            _check(self.lib.bz2b200_engine_create_batch(C.byref(self.h), device, level, window_bytes, max_items),
+                   "engine_create_batch")
+        else:
+            _check(self.lib.bz2b200_engine_create(C.byref(self.h), device, level, window_bytes), "engine_create")
 
     def close(self):
         if self.h:
@@ -187,6 +210,52 @@ class Engine:
                "compress_device")
         self.stats = st
         return out_len.value
+
+    def compress_batch_raw(self, src, offsets, dst_cap=None, flags=0):
+        """One bz2b200_compress_batch_host call on a flat uint8 array and its item offsets (n+1, offsets[0] = 0).
+        Returns (rc, dst array, out_offsets, stream_crcs); raises only when the library is missing."""
+        src = np.ascontiguousarray(src, np.uint8)
+        offs = np.ascontiguousarray(offsets, np.uint64)
+        n = offs.size - 1
+        if dst_cap is None:
+            dst_cap = sum(compress_bound(self.level, int(x)) for x in np.diff(offs))
+        dst = np.empty(max(dst_cap, 1), np.uint8)
+        out_offs = np.zeros(n + 1, np.uint64)
+        crcs = np.zeros(max(n, 1), np.uint32)
+        st = Stats()
+        rc = self.lib.bz2b200_compress_batch_host(self.h, _ptr(src), _u64p(offs), n, dst.ctypes.data, dst_cap,
+                                                  _u64p(out_offs), crcs.ctypes.data_as(C.POINTER(C.c_uint32)), flags,
+                                                  C.byref(st))
+        self.stats = st
+        return rc, dst, out_offs, crcs[:n]
+
+    def compress_batch(self, items, flags=0):
+        """Compress every item to its own complete .bz2 stream in one call (bz2b200_compress_batch_host)."""
+        arrs = [np.frombuffer(x, dtype=np.uint8) if isinstance(x, (bytes, bytearray)) else np.ascontiguousarray(x, np.uint8)
+                for x in items]
+        offs = np.zeros(len(arrs) + 1, np.uint64)
+        offs[1:] = np.cumsum([a.size for a in arrs], dtype=np.uint64)
+        src = np.concatenate(arrs) if arrs else np.zeros(0, np.uint8)
+        rc, dst, out_offs, crcs = self.compress_batch_raw(src, offs, flags=flags)
+        _check(rc, "compress_batch_host")
+        self.stream_crcs = crcs
+        return [dst[int(out_offs[k]):int(out_offs[k + 1])].tobytes() for k in range(len(arrs))]
+
+    def compress_batch_device(self, d_src_ptr, offsets, d_dst_ptr, dst_cap, flags=0, stream_crcs=None):
+        """Device input and output (e.g. torch tensor .data_ptr()); offsets: host array of n+1 item offsets.
+        Returns the numpy array of n+1 stream offsets in the destination."""
+        offs = np.ascontiguousarray(offsets, np.uint64)
+        n = offs.size - 1
+        out_offs = np.zeros(n + 1, np.uint64)
+        crcp = None
+        if stream_crcs is not None:
+            assert stream_crcs.dtype == np.uint32 and stream_crcs.size >= n
+            crcp = stream_crcs.ctypes.data_as(C.POINTER(C.c_uint32))
+        st = Stats()
+        _check(self.lib.bz2b200_compress_batch_device(self.h, d_src_ptr, _u64p(offs), n, d_dst_ptr, dst_cap, _u64p(out_offs),
+                                                      crcp, flags, C.byref(st)), "compress_batch_device")
+        self.stats = st
+        return out_offs
 
     def fetch(self, name, dtype, count=None):
         cap = (1 << 28)

@@ -25,6 +25,7 @@
 #include <sys/stat.h>
 #include <unistd.h>
 #include <time.h>
+#include <stdint.h>
 
 enum { OP_COMPRESS, OP_DECOMPRESS, OP_TEST };
 static int level = 9, to_stdout = 0, keep = 0, force = 0, quiet = 0, verbose = 0, small = 0, op = OP_COMPRESS;
@@ -288,7 +289,149 @@ static void report(const char* name, unsigned long long nin, unsigned long long 
            (double)nin / (double)nout, 8.0 * (double)nout / (double)nin, 100.0 * (1.0 - (double)nout / (double)nin), nin, nout);
 }
 
+/* Consecutive small regular files are compressed together: one bz2b200_compress_batch_host call per batch of up to
+ * BATCH_BYTES of input or BATCH_FILES files, on one engine kept for the invocation, instead of a whole set of kernel
+ * launches and host round trips per file.  Every file still becomes its own stream with the bytes a call of its own
+ * gives.  The batch is finished -- files written, closed, chmod-ed, removed unless -k, reported -- in argument order,
+ * and before anything is printed about a later file or a later file is handled another way, so stderr and the output
+ * files keep the order of one file at a time.  Not used with -vv and above (the per-block trace) or under
+ * BZ2_B200_CLI_STREAM=1. */
+#define BATCH_BYTES ((size_t)32 << 20)
+#define BATCH_FILES 1024
+static struct {
+   unsigned char* buf; size_t len, cap;
+   int n;
+   char* name[BATCH_FILES];
+   mode_t mode[BATCH_FILES];
+   uint64_t offs[BATCH_FILES + 1];
+} pend;
+static struct { bz2b200_engine* e; int level; } batch_eng;
+static int full_batch_rc;          /* exit code of batches flushed because they were full */
+
+static int batch_usable(void)
+{
+   const char* force_stream = getenv("BZ2_B200_CLI_STREAM");
+   return verbose < 2 && !(force_stream && *force_stream == '1');
+}
+
+/* Compress and finish every pending file.  Returns the largest exit code among them. */
+static int flush_batch(void)
+{
+   const int lvl = small && level > 2 ? 2 : level;
+   int rc = 0, k, r;
+   size_t cap = 0;
+   unsigned char* dst;
+   uint64_t out_offs[BATCH_FILES + 1];
+   if (pend.n == 0) return 0;
+   for (k = 0; k < pend.n; k++) cap += bz2b200_compress_bound(lvl, (size_t)(pend.offs[k + 1] - pend.offs[k]));
+   dst = (unsigned char*)malloc(cap ? cap : 1);
+   if (batch_eng.e && batch_eng.level != lvl) { bz2b200_engine_destroy(batch_eng.e); batch_eng.e = NULL; }
+   r = !dst ? BZ2B200_ENOMEM
+       : batch_eng.e ? 0
+       : bz2b200_engine_create_batch(&batch_eng.e, getenv("BZ2_B200_DEVICE") ? atoi(getenv("BZ2_B200_DEVICE")) : 0, lvl,
+                                     BATCH_BYTES, BATCH_FILES);
+   if (r == 0) {
+      batch_eng.level = lvl;
+      bz2b200_engine_set_verbosity(batch_eng.e, verbose);
+      r = bz2b200_compress_batch_host(batch_eng.e, pend.buf, pend.offs, (size_t)pend.n, dst, cap, out_offs, NULL,
+                                      BZ2B200_TAIL_STREAMED, NULL);
+   }
+   for (k = 0; k < pend.n; k++) {
+      const char* name = pend.name[k];
+      const unsigned long long nin = pend.offs[k + 1] - pend.offs[k];
+      unsigned long long nout;
+      char outname[4096];
+      FILE* out;
+      if (r) {
+         fprintf(stderr, "%s: %s: the GPU compressor failed (%d: %s)%s\n", prog, name, r, bz2b200_last_error(),
+                 r == BZ2B200_ENODEV ? "; this build has no CPU path" : "");
+         rc = 1;
+         continue;
+      }
+      nout = out_offs[k + 1] - out_offs[k];
+      if (to_stdout) {
+         if (fwrite(dst + out_offs[k], 1, nout, stdout) != nout || fflush(stdout) != 0) {
+            fprintf(stderr, "%s: write error: %s\n", prog, strerror(errno));
+            rc = 1;
+            continue;
+         }
+         report(name, nin, nout);
+         continue;
+      }
+      snprintf(outname, sizeof outname, "%s.bz2", name);
+      out = fopen(outname, "wb");
+      if (!out) { fprintf(stderr, "%s: Can't create output file %s: %s.\n", prog, outname, strerror(errno)); rc = 1; continue; }
+      if (fwrite(dst + out_offs[k], 1, nout, out) != nout || fflush(out) != 0) {
+         fprintf(stderr, "%s: write error: %s\n", prog, strerror(errno));
+         fclose(out);
+         remove(outname);
+         rc = 1;
+         continue;
+      }
+      if (fclose(out) != 0) { remove(outname); rc = 1; continue; }
+      chmod(outname, pend.mode[k] & 07777);
+      if (!keep) remove(name);
+      report(name, nin, nout);
+   }
+   free(dst);
+   for (k = 0; k < pend.n; k++) free(pend.name[k]);
+   pend.n = 0; pend.len = 0;
+   return rc;
+}
+
+/* Queue `name` for the next batch if it is a small regular file that would be compressed without a word on stderr.
+ * 1: queued; 0: the caller flushes the batch and handles the file one at a time. */
+static int queue_small_file(const char* name)
+{
+   struct stat st;
+   size_t L = strlen(name), size, got;
+   FILE* in;
+   char outname[4096];
+   int k;
+   if (!batch_usable() || L + 5 > sizeof outname || stat(name, &st) != 0 || !S_ISREG(st.st_mode)) return 0;
+   if ((unsigned long long)st.st_size > SMALL_FILE) return 0;
+   if (L > 4 && strcmp(name + L - 4, ".bz2") == 0 && !force) return 0;
+   snprintf(outname, sizeof outname, "%s.bz2", name);
+   if (!to_stdout && !force && access(outname, F_OK) == 0) return 0;
+   size = (size_t)st.st_size;
+   for (k = 0; k < pend.n; k++) if (!strcmp(pend.name[k], name)) return 0;          /* the same file twice */
+   if (pend.n == BATCH_FILES || pend.len + size > BATCH_BYTES) { const int r = flush_batch(); if (r > full_batch_rc) full_batch_rc = r; }
+   if (pend.len + size > pend.cap) {
+      size_t nc = pend.cap ? pend.cap : ((size_t)1 << 20);
+      unsigned char* nb;
+      while (nc < pend.len + size) nc *= 2;
+      nb = (unsigned char*)realloc(pend.buf, nc);
+      if (!nb) return 0;
+      pend.buf = nb; pend.cap = nc;
+   }
+   in = fopen(name, "rb");
+   if (!in) return 0;
+   got = fread(pend.buf + pend.len, 1, size, in);
+   if (ferror(in) || got != size || fgetc(in) != EOF) { fclose(in); return 0; }    /* the file changed: one at a time */
+   fclose(in);
+   pend.name[pend.n] = strdup(name);
+   if (!pend.name[pend.n]) return 0;
+   pend.mode[pend.n] = st.st_mode;
+   pend.offs[pend.n] = pend.len;
+   pend.len += size;
+   pend.n++;
+   pend.offs[pend.n] = pend.len;
+   return 1;
+}
+
+static int do_file_now(const char* name);
+
 static int do_file(const char* name)
+{
+   int r, r2;
+   if (op != OP_COMPRESS) return expand_file(name);
+   if (queue_small_file(name)) return 0;
+   r = flush_batch();
+   r2 = do_file_now(name);
+   return r > r2 ? r : r2;
+}
+
+static int do_file_now(const char* name)
 {
    char outname[4096];
    struct stat st;
@@ -296,7 +439,6 @@ static int do_file(const char* name)
    unsigned long long nin = 0, nout = 0;
    int rc;
    size_t L = strlen(name);
-   if (op != OP_COMPRESS) return expand_file(name);
    if (L + 5 > sizeof outname) { fprintf(stderr, "%s: file name too long: %s\n", prog, name); return 1; }
    if (stat(name, &st) != 0) { fprintf(stderr, "%s: Can't open input file %s: %s.\n", prog, name, strerror(errno)); return 1; }
    if (S_ISDIR(st.st_mode)) { fprintf(stderr, "%s: Input file %s is a directory.\n", prog, name); return 1; }
@@ -415,7 +557,8 @@ static int run(int argc, char** argv)
       if (!dashdash && argv[i][0] == '-' && argv[i][1]) continue;
       { int r = do_file(argv[i]); if (r > rc) rc = r; }
    }
-   return rc;
+   { int r = flush_batch(); if (r > rc) rc = r; }
+   return rc > full_batch_rc ? rc : full_batch_rc;
 }
 
 /* Everything is flushed and closed by the time run() returns; leaving through _exit skips the CUDA

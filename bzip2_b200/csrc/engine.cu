@@ -51,7 +51,8 @@ void engine_free(EngineFull* e)
                    e->pre, e->prebits, e->ngroups, e->d_in, e->d_out,
                    e->bt.X, e->bt.P, e->bt.crc, e->bt.origptr, e->bt.power_q, e->bt.inuse, e->bt.ninuse, e->bt.nmtf,
                    e->bt.mtffreq, e->bt.bits, e->bt.bitoff, e->lists.counts[0], e->lists.counts[1],
-                   e->tie_tmp, e->bt.tie_flag, e->bt.tie_lo };
+                   e->tie_tmp, e->bt.tie_flag, e->bt.tie_lo,
+                   e->it.start, e->it.enc, e->it.cnt, e->it.first, e->it.byteoff, e->it.crc };
    for (void* p : dev) if (p) cudaFree(p);
    for (int w = 0; w < 2; w++) {
       for (int c = 0; c < N_SMALL_CLASSES; c++) if (e->lists.small_items[w][c]) cudaFree(e->lists.small_items[w][c]);
@@ -61,6 +62,7 @@ void engine_free(EngineFull* e)
    if (e->h_counts) cudaFreeHost(e->h_counts);
    if (e->h_blk) cudaFreeHost(e->h_blk);
    if (e->h_trace) cudaFreeHost(e->h_trace);
+   if (e->h_items) cudaFreeHost(e->h_items);
    if (e->h_in) cudaFreeHost(e->h_in);
    if (e->h_out) cudaFreeHost(e->h_out);
    if (e->d_in2) cudaFree(e->d_in2);
@@ -73,7 +75,7 @@ void engine_free(EngineFull* e)
    free(e);
 }
 
-int engine_new(EngineFull** out, int device, int level, size_t window_bytes, bool bounded)
+int engine_new(EngineFull** out, int device, int level, size_t window_bytes, bool bounded, size_t extra_slots)
 {
    int ndev = 0;
    cudaError_t ce = cudaGetDeviceCount(&ndev);
@@ -110,6 +112,8 @@ int engine_new(EngineFull** out, int device, int level, size_t window_bytes, boo
    e->win_cap = (u32)window_bytes;
    e->enc_cap = (u32)(window_bytes + window_bytes / 4 + 4096);
    e->blk_cap = e->enc_cap / e->nmax + 2;
+   // batch engines: one slot more per item a window may hold (every item, however small, ends its own block)
+   e->blk_cap = (u32)((size_t)e->blk_cap + (extra_slots < MAX_BLOCKS ? extra_slots : MAX_BLOCKS));
    if (e->blk_cap > MAX_BLOCKS) e->blk_cap = MAX_BLOCKS;
    {
       const size_t E = e->enc_cap, B = e->blk_cap;
@@ -136,6 +140,7 @@ int engine_new(EngineFull** out, int device, int level, size_t window_bytes, boo
       ALLOC(e->bwt, E + 64); ALLOC(e->z, E + 64); ALLOC(e->mtfv, E + B + 64);
       u32 hist_log2 = 18;
       { const char* hl = getenv("BZ2_B200_HIST_LOG2"); if (hl) { const int v = atoi(hl); if (v >= 16 && v <= 22) hist_log2 = (u32)v; } }
+      e->hist_log2 = hist_log2;
       e->hist_stride = 1u << 16;
       while (e->hist_stride < (1u << hist_log2) && e->hist_stride < e->nmax / 4) e->hist_stride <<= 1;
       if (hist_log2 > 18 && e->hist_stride < e->nmax * 2u) e->hist_stride = 1u << hist_log2;
@@ -510,7 +515,7 @@ static void feed_shutdown(EngineFull* e)
 }
 
 // a new stream starts: wait for a window the previous (abandoned) stream may still have in flight, then forget it
-static void feed_reset(EngineFull* e)
+void feed_reset(EngineFull* e)
 {
    AsyncFeed& a = e->af;
    if (!a.inited) return;

@@ -60,6 +60,16 @@ struct BlockTables {                        // per-window block metadata (device
    u64* bitoff;     // [nb+1] absolute stream bit offset of each block
 };
 
+// Batch windows (batch.cu): many independent inputs packed into one window, each becoming its own stream.
+struct ItemTables {                         // device arrays, [blk_cap + 1] or [blk_cap]
+   u32* start;      // [n+1] window-relative input start of each item (start[n] = W)
+   u32* enc;        // [n]   encoded start of each item
+   u32* cnt;        // [n]   blocks of each item
+   u32* first;      // [n+1] first block of each item (first[n] = blocks of the window)
+   u64* byteoff;    // [n+1] byte offset of each item's stream in the window's output (byteoff[n] = window bytes)
+   u32* crc;        // [n]   combined CRC of each item's stream
+};
+
 struct Engine;
 
 // One shard's chunk structure for the multi-GPU boundary chain (stage1_rle.cu)
@@ -79,11 +89,16 @@ int scan_boundary(ScanState* s, u32 start, u32 limit, u32 tail_merge, u32* bound
 
 // ---- stage launchers (each returns 0 or a negative error; all work on e->stream) ----
 int stage1_run(Engine* e, const u8* d_in, u32 W, bool is_final, bool tail_merge, u32* nb_out, u32* consumed_out, u32* enc_total_out);
+int stage1_items_run(Engine* e, const u8* d_in, u32 W, u32 n_items, u32 nb_ub, bool tail_merge,
+                     u32* nb_out, u32* enc_total_out, u32* max_blk_out);
 int stage2_init();
-int stage2_run(Engine* e, u32 nb, u32 E);
+int stage2_run(Engine* e, u32 nb, u32 E, u32 max_blk = 0);
+u32 s2_batch_stride(const Engine* e, u32 max_blk);
 int stage2_power_origptr(Engine* e, u32 b0, u32 g);
 int stage3_run(Engine* e, u32 nb, u32 E);
-int stage4_run(Engine* e, u32 nb, u32 E, u8* d_out, u64 origin_bit, u64 start_bit, u64* end_bit_out);
+// n_items != 0: a batch window; blocks are framed per item (e->it) from bit 0 and origin_bit / start_bit are unused
+int stage4_run(Engine* e, u32 nb, u32 E, u8* d_out, u64 origin_bit, u64 start_bit, u64* end_bit_out, u32 n_items = 0);
+int stage4_empty_items(Engine* e, u32 n_items, u8* d_out, u64* end_bit_out);
 int put_bits_device(Engine* e, u8* d_out, u64 origin_bit, u64 bitpos, u64 value, int nbits);
 int concat_bits_device(u8* d_dst, u64 dst_bit, const u8* d_src, u64 nbits);
 
@@ -111,6 +126,7 @@ struct Engine {
    u32 *hist;
    u32 s2_group;           // blocks sorted per BWT sub-batch (0 = whole window)
    u32 hist_stride;        // k-gram bins reserved per block (power of two, 2^16..2^18)
+   u32 hist_log2;          // the k-gram budget asked for (BZ2_B200_HIST_LOG2, default 18)
    u8  *code;              // [blk_cap*256]
    u32 *kk, *nbins, *hh, *kbits, *ksym;   // [blk_cap]
    u64 *K, *kscrA, *kscrB; // [E] packed text keys; 64-bit key scratch of the large path
@@ -130,6 +146,7 @@ struct Engine {
    u32 tie_force;          // BZ2_B200_TIE_FORCE=1: replay every exact-power block (tests: closed form == replay)
    SegLists lists;
    BlockTables bt;
+   ItemTables it;          // allocated by the first batch call
 
    // stage-1 tile scratch
    u32 *tile_len, *tile_ext, *tile_carry, *tile_size, *tile_base;

@@ -49,13 +49,15 @@ struct EngineFull : Engine {
    cudaEvent_t ev_h2d[2];
    void (*after_s1)(EngineFull*, u32 consumed, void* ctx);
    void* after_s1_ctx;
+   u32* h_items;               // batch calls: pinned [4 * (blk_cap + 1)] u32 -- item starts, first blocks, CRCs, byte offsets
 };
 
 // engine.cu
-int  engine_new(EngineFull** out, int device, int level, size_t window_bytes, bool bounded = false);
+int  engine_new(EngineFull** out, int device, int level, size_t window_bytes, bool bounded = false, size_t extra_slots = 0);
 void engine_free(EngineFull* e);
 int  ensure_staging(EngineFull* e, bool need_hin);
 void stream_reset(EngineFull* e);
+void feed_reset(EngineFull* e);
 int  run_window(EngineFull* e, const u8* d_in, u32 W, bool is_final, bool tail_merge,
                 u8* d_out, u64 origin_bit, u32* consumed, u32* nb_out);
 int  set_err(int code, const char* msg);

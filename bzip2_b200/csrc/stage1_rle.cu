@@ -76,6 +76,7 @@ struct S1Params {
    u32 prev_byte;       // byte before in[0] (256: none) and the length of the run it ends,
    u32 carry0;          // when the window does not start at a chunk boundary (shard scans)
    const u32* Q; u32* EQ;                // LOCATE mode: input positions Q[k] -> encoded offsets EQ[k]
+   const u32* seams; u32 nseams;         // batch windows: sorted item starts; no run continues into one (0: none)
 };
 
 template <int MODE>
@@ -132,6 +133,16 @@ __global__ void __launch_bounds__(S1_THREADS) k_tile(S1Params p)
    if (pos0 >= 1 && pos0 - 1 < (i64)p.W) prevb = p.in[pos0 - 1];
    else if (pos0 == 0) prevb = p.prev_byte;
    if (pos0 + S1_BPT >= 0 && pos0 + S1_BPT < (i64)p.W) nextb = p.in[pos0 + S1_BPT];
+   // Batch windows hold many independent inputs: an item start behaves like a window start (the byte before it is
+   // "none"), so no run, chunk or block crosses from one item into the next and the last byte of every item ends a chunk.
+   u32 seam = 0;                                            // bit k: position pos0 + k starts an item (k = 0..16)
+   if (p.nseams) {
+      u32 lo = 0, hi = p.nseams;
+      while (lo < hi) { const u32 mid = (lo + hi) >> 1; if ((i64)p.seams[mid] < pos0) lo = mid + 1; else hi = mid; }
+      for (u32 s = lo; s < p.nseams && (i64)p.seams[s] <= pos0 + S1_BPT; s++) seam |= 1u << (u32)((i64)p.seams[s] - pos0);
+      if (seam & 1u) prevb = 256;
+      if (seam & (1u << S1_BPT)) nextb = 256;
+   }
 
    // per-position "continues the run" flags and the thread aggregate
    u32 eqmask = 0, vmask = 0;
@@ -142,6 +153,7 @@ __global__ void __launch_bounds__(S1_THREADS) k_tile(S1Params p)
       bool valid = (q >= 0 && q < (i64)p.W);
       u32 pb = (k == 0) ? prevb : (u32)c[k - 1];
       if (k > 0 && q == 0) pb = p.prev_byte;               // 256 unless the window continues a run (shard scans)
+      if ((seam >> k) & 1u) pb = 256;
       bool eq = valid && (pb == (u32)c[k]);
       if (valid) {
          vmask |= 1u << k;
@@ -212,7 +224,8 @@ __global__ void __launch_bounds__(S1_THREADS) k_tile(S1Params p)
       const u32 jj = ph[k];
       const i64 q = pos0 + k;
       const u32 ch = c[k];
-      const u32 nb_ = (k == 15) ? nextb : (((vmask >> (k + 1)) & 1) ? (u32)c[k + 1] : 256u);
+      // the next byte continues this run iff its flag says so (an item start never does: the item ends here)
+      const u32 nb_ = (k == 15) ? nextb : (((eqmask >> (k + 1)) & 1) ? ch : 256u);
       bool last = (jj == 254);
       if (q == (i64)p.W - 1) last = last || (p.is_final != 0);
       else last = last || (nb_ != ch);
@@ -517,7 +530,7 @@ int stage1_run(Engine* e, const u8* d_in, u32 W, bool is_final, bool tail_merge,
    p.tile_len = e->tile_len; p.tile_ext = e->tile_ext; p.tile_carry = e->tile_carry;
    p.tile_size = e->tile_size; p.tile_base = e->tile_base;
    p.enc = e->enc; p.cend = e->cend; p.X = e->bt.X; p.P = e->bt.P; p.nb_find = 0; p.scalars = e->s1_scalars;
-   p.prev_byte = 256; p.carry0 = 0; p.Q = nullptr; p.EQ = nullptr;
+   p.prev_byte = 256; p.carry0 = 0; p.Q = nullptr; p.EQ = nullptr; p.seams = nullptr; p.nseams = 0;
 
    // One host round trip per window: everything below is sized by upper bounds (RLE1 grows the data by at most 5/4,
    // a block holds at least nmax encoded bytes) and reads the actual counts from device memory.
@@ -574,6 +587,87 @@ int stage1_run(Engine* e, const u8* d_in, u32 W, bool is_final, bool tail_merge,
    return 0;
 }
 
+// ---- batch windows: many independent inputs, each its own stream ---------------------------------
+// k_chain's walk, one warp per item, over the item's encoded range [enc[i], enc[i+1]) as a final range (every item is a
+// whole stream).  COUNT: the item's block count -> cnt[i] and the largest block -> scalars[5].  WRITE: block ends -> X
+// from the item's first block (first[] = exclusive scan of cnt); item 0 also publishes the window's block count.
+template <bool WRITE>
+__global__ void __launch_bounds__(256) k_chain_items(const u8* cend, const u32* enc, u32 n_items, u32* scalars, u32 nmax,
+                                                     u32 tail_merge, u32* cnt, const u32* first, u32* X)
+{
+   const u32 l = lane_id();
+   const u32 i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+   if (i >= n_items) return;
+   const u32 Etot = scalars[2];
+   const u32 Ee = (i + 1 < n_items) ? enc[i + 1] : Etot;
+   u32 x = enc[i], nb = 0, mx = 0;
+   const u32 base = WRITE ? first[i] : 0;
+   if (WRITE && i == 0 && l == 0) { X[0] = 0; scalars[0] = first[n_items]; scalars[1] = Etot; }
+   while (x < Ee) {
+      const u32 target = x + nmax - 1;
+      u32 nx = Ee;
+      if (target < Ee) {
+         const u32 e = target + l;
+         const bool f = (l < 8) && (e < Ee) && (cend[e] != 0);
+         const u32 m = __ballot_sync(FULL, f);
+         if (m) {
+            nx = target + (u32)(__ffs(m) - 1) + 1;
+            if (tail_merge && Ee - nx == 1) nx = Ee;
+         }
+      }
+      nb++;
+      if (WRITE && l == 0) X[base + nb] = nx;
+      mx = max(mx, nx - x);
+      x = nx;
+   }
+   if (!WRITE && l == 0) { cnt[i] = nb; if (mx) atomicMax(&scalars[5], mx); }
+}
+
+// Stage 1 of a batch window: e->it.start[0, n_items) holds the window-relative item starts.  Blocks never cross an item
+// start; X, P and crc come out as for a single stream, and it.first[i] is item i's first block.
+int stage1_items_run(Engine* e, const u8* d_in, u32 W, u32 n_items, u32 nb_ub, bool tail_merge,
+                     u32* nb_out, u32* enc_total_out, u32* max_blk_out)
+{
+   cudaStream_t st = e->stream;
+   const u32 align = (u32)((uintptr_t)d_in & 15);
+   const u32 ntiles = (W + align + S1_TILE - 1) / S1_TILE;
+   const u32 Eub = W + W / 4 + 64;
+   if (Eub > e->enc_cap || nb_ub > e->blk_cap || n_items == 0 || n_items > e->blk_cap) {
+      snprintf(e->err, sizeof e->err, "batch window too large for the engine (%u bytes, %u items)", W, n_items);
+      return -3;
+   }
+   S1Params p;
+   p.in = d_in; p.W = W; p.is_final = 1;
+   p.tile_len = e->tile_len; p.tile_ext = e->tile_ext; p.tile_carry = e->tile_carry;
+   p.tile_size = e->tile_size; p.tile_base = e->tile_base;
+   p.enc = e->enc; p.cend = e->cend; p.X = e->bt.X; p.P = e->bt.P; p.nb_find = 1; p.scalars = e->s1_scalars;
+   p.prev_byte = 256; p.carry0 = 0; p.Q = e->it.start; p.EQ = e->it.enc;
+   p.seams = e->it.start; p.nseams = n_items;
+   BZ_CUDA(e, cudaMemsetAsync(e->s1_scalars + 5, 0, sizeof(u32), st));
+   k_tile<S1_AGG><<<ntiles, S1_THREADS, 0, st>>>(p);                                   BZ_KCHECK(e);
+   k_scan_runs<<<1, 1024, 0, st>>>(e->tile_len, e->tile_ext, e->tile_carry, ntiles, 0);   BZ_KCHECK(e);
+   k_tile<S1_COUNT><<<ntiles, S1_THREADS, 0, st>>>(p);                                 BZ_KCHECK(e);
+   k_scan_u32<<<1, 1024, 0, st>>>(e->tile_size, e->tile_base, ntiles, e->s1_scalars + 2); BZ_KCHECK(e);
+   BZ_CUDA(e, cudaMemsetAsync(e->cend, 0, (size_t)Eub + 16, st));
+   k_tile<S1_SCATTER><<<ntiles, S1_THREADS, 0, st>>>(p);                               BZ_KCHECK(e);
+   k_tile<S1_LOCATE><<<n_items, S1_THREADS, 0, st>>>(p);                               BZ_KCHECK(e);
+   const u32 cgrid = (n_items + 7) / 8;
+   k_chain_items<false><<<cgrid, 256, 0, st>>>(e->cend, e->it.enc, n_items, e->s1_scalars, e->nmax, tail_merge ? 1 : 0,
+                                               e->it.cnt, nullptr, nullptr);        BZ_KCHECK(e);
+   k_scan_u32<<<1, 1024, 0, st>>>(e->it.cnt, e->it.first, n_items, e->it.first + n_items); BZ_KCHECK(e);
+   k_chain_items<true><<<cgrid, 256, 0, st>>>(e->cend, e->it.enc, n_items, e->s1_scalars, e->nmax, tail_merge ? 1 : 0,
+                                              nullptr, e->it.first, e->bt.X);       BZ_KCHECK(e);
+   BZ_CUDA(e, cudaMemsetAsync(e->bt.P, 0, sizeof(u32), st));
+   k_tile<S1_FIND><<<nb_ub, S1_THREADS, 0, st>>>(p);                                   BZ_KCHECK(e);
+   BZ_CUDA(e, cudaMemcpyAsync(e->h_scalars, e->s1_scalars, 6 * sizeof(u32), cudaMemcpyDeviceToHost, st));
+   BZ_CUDA(e, cudaEventRecord(e->ev_s1, st));
+   BZ_CUDA(e, cudaMemsetAsync(e->bt.crc, 0, sizeof(u32) * nb_ub, st));
+   k_crc<<<dim3(CRC_CTAS_PER_BLOCK, nb_ub), CRC_THREADS, 0, st>>>(d_in, e->bt.P, e->bt.crc, e->s1_scalars); BZ_KCHECK(e);
+   k_crc_final<<<(nb_ub + 255) / 256, 256, 0, st>>>(e->bt.crc, e->s1_scalars);            BZ_KCHECK(e);
+   BZ_CUDA(e, cudaEventSynchronize(e->ev_s1));
+   *nb_out = e->h_scalars[0]; *enc_total_out = e->h_scalars[1]; *max_blk_out = e->h_scalars[5];
+   return 0;
+}
 
 // ---- shard scan (multi-GPU sharding of one stream by block, SURVEY 8e) ---------------------------
 // The chunk structure of a shard (cend flags, encoded offsets) does not depend on where blocks

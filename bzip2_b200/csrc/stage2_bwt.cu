@@ -1423,14 +1423,26 @@ int stage2_init()
    return c == cudaSuccess ? 0 : -1;
 }
 
-int stage2_run(Engine* e, u32 nb, u32 E)
+// max_blk = 0: a single-stream window (blocks of up to nmax + 16 bytes, e->hist_stride k-gram bins per block).
+// Batch windows pass their largest block: the k-gram budget is the one engine_new picks for an nmax of that size,
+// never below 2^16 bins (the tie-order replay uses each slot as its 65,536-entry bucket table, stage2_tie.cu), and
+// the per-block grids are sized by that block, so a window of many small blocks does not clear and scan full slots.
+u32 s2_batch_stride(const Engine* e, u32 max_blk)
+{
+   u32 s = 1u << 16;
+   while (s < (1u << e->hist_log2) && s < max_blk / 4) s <<= 1;
+   if (e->hist_log2 > 18 && s < max_blk * 2u) s = 1u << e->hist_log2;
+   return s < e->hist_stride ? s : e->hist_stride;
+}
+
+int stage2_run(Engine* e, u32 nb, u32 E, u32 max_blk)
 {
    cudaStream_t st = e->stream;
    S2Params p;
    p.T = e->enc; p.X = e->bt.X; p.nb = nb;
    p.sa = e->sa; p.rank = e->rank;
    p.keyA = e->keyA; p.keyB = e->keyB; p.idxB = e->idxB;
-   p.hist = e->hist; p.hist_stride = e->hist_stride; p.code = e->code; p.kk = e->kk; p.nbins = e->nbins;
+   p.hist = e->hist; p.hist_stride = max_blk ? s2_batch_stride(e, max_blk) : e->hist_stride; p.code = e->code; p.kk = e->kk; p.nbins = e->nbins;
    p.hh = e->hh; p.kbits = e->kbits; p.ksym = e->ksym; p.K = e->K; p.kscrA = e->kscrA; p.kscrB = e->kscrB;
    p.debug = trace_on() ? 1 : 0;
    p.kg_agg_alpha = KG_AGG_MAX_ALPHA;
@@ -1443,13 +1455,13 @@ int stage2_run(Engine* e, u32 nb, u32 E)
    BZ_CUDA(e, cudaMemsetAsync(e->bt.inuse, 0, (size_t)nb * 256, st));
    BZ_CUDA(e, cudaMemsetAsync(e->bt.power_q, 0, sizeof(u32) * nb, st));
    BZ_CUDA(e, cudaMemsetAsync(e->s1_scalars + 4, 0, sizeof(u32), st));
-   const u32 max_n = e->nmax + 16;
+   const u32 max_n = (max_blk ? max_blk : e->nmax) + 16;
    // Blocks are sorted in sub-batches small enough for their rank/sa arrays to stay in L2.
    const u32 group = e->s2_group ? e->s2_group : nb;
    for (u32 b0 = 0; b0 < nb; b0 += group) {
       const u32 g = (nb - b0 < group) ? (nb - b0) : group;
       p.b0 = b0;
-      BZ_CUDA(e, cudaMemsetAsync(e->hist, 0, (size_t)g * e->hist_stride * sizeof(u32), st));
+      BZ_CUDA(e, cudaMemsetAsync(e->hist, 0, (size_t)g * p.hist_stride * sizeof(u32), st));
       BZ_CUDA(e, cudaMemsetAsync(e->lists.counts[0], 0, sizeof(u32) * N_CLASSES, st));
       const dim3 gtiles((max_n + KG_TILE - 1) / KG_TILE, g);
       k_inuse<<<gtiles, KG_THREADS, 0, st>>>(p);                                                BZ_KCHECK(e);
@@ -1459,7 +1471,7 @@ int stage2_run(Engine* e, u32 nb, u32 E)
       k_kgram<KG_HISTOFF, true><<<gtiles, KG_THREADS, 0, st>>>(p);                              BZ_KCHECK(e);
       k_kgram_scan<<<g, 1024, 0, st>>>(p);                                                      BZ_KCHECK(e);
       k_kgram<KG_PLACE, false><<<gtiles, KG_THREADS, 0, st>>>(p);                                      BZ_KCHECK(e);
-      k_seg_init<<<dim3((e->hist_stride + 255) / 256, g), 256, 0, st>>>(p, lists_dev(e, 0));    BZ_KCHECK(e);
+      k_seg_init<<<dim3((p.hist_stride + 255) / 256, g), 256, 0, st>>>(p, lists_dev(e, 0));    BZ_KCHECK(e);
       dbg_sync(e, "k-gram phase");
 
       int cur = 0;

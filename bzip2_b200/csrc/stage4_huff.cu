@@ -545,6 +545,95 @@ int concat_bits_stream(u8* d_dst, u64 dst_bit, const u8* d_src, u64 nbits, cudaS
    return cudaGetLastError() == cudaSuccess ? 0 : -1;
 }
 
+// ---- batch windows: every item is its own stream ------------------------------------------------
+// Item i's stream is 32 header bits, its blocks in order, 80 trailer bits and padding to a byte (compress.c:841-845,
+// :874-879); the streams are laid back to back from bit 0.  One CTA: the byte length of every item, their exclusive scan
+// -> ibyte[0..n] (ibyte[n] = bytes of the window), and the bit offset of every block inside its item's stream.
+__global__ void __launch_bounds__(1024) k_item_offsets(const u64* bits, u64* bitoff, const u32* first, u32 n, u64* ibyte)
+{
+   __shared__ u64 wsum[32];
+   __shared__ u64 s_run;
+   if (threadIdx.x == 0) s_run = 0;
+   __syncthreads();
+   const u32 l = lane_id(), w = threadIdx.x >> 5;
+   for (u32 base = 0; base < n; base += 1024) {
+      const u32 i = base + threadIdx.x;
+      u64 v = 0;
+      if (i < n) {
+         u64 nbits = 32 + 80;
+         for (u32 b = first[i]; b < first[i + 1]; b++) nbits += bits[b];
+         v = (nbits + 7) >> 3;
+      }
+      u64 inc = v;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) { const u64 q = __shfl_up_sync(FULL, inc, d); if (l >= (u32)d) inc += q; }
+      if (l == 31) wsum[w] = inc;
+      __syncthreads();
+      u64 pre = s_run;
+      for (u32 k = 0; k < w; k++) pre += wsum[k];
+      if (i < n) {
+         const u64 off = pre + inc - v;
+         ibyte[i] = off;
+         u64 bp = off * 8 + 32;
+         for (u32 b = first[i]; b < first[i + 1]; b++) { bitoff[b] = bp; bp += bits[b]; }
+      }
+      __syncthreads();
+      if (threadIdx.x == 1023) s_run = pre + inc;
+      __syncthreads();
+   }
+   if (threadIdx.x == 0) { ibyte[n] = s_run; bitoff[first[n]] = s_run * 8; }
+}
+
+__device__ void put_bits_or(u32* outw, u64 bitpos, u64 value, int nbits)
+{
+   for (int done = 0; done < nbits;) {
+      const u64 bp = bitpos + done;
+      const u32 sh = (u32)(bp & 31);
+      const int take = min(32 - (int)sh, nbits - done);
+      const u32 chunk = (u32)((value >> (nbits - done - take)) & ((take == 32) ? 0xffffffffu : ((1u << take) - 1u)));
+      atomicOr(&outw[bp >> 5], bswap32(chunk << (32 - sh - take)));
+      done += take;
+   }
+}
+
+// One thread per item: the "BZh<level>" header, and the trailer with the combined CRC of the item's blocks
+// (compress.c:826-828).  An empty item is header and trailer only.  Runs after k_pack: headers and trailers are ORed
+// into words the neighbouring streams share.
+__global__ void __launch_bounds__(256) k_item_frames(u32* outw, const u64* ibyte, const u64* bits, const u32* first,
+                                                     const u32* crc, u32* icrc, u32 n, u32 level)
+{
+   const u32 i = blockIdx.x * 256 + threadIdx.x;
+   if (i >= n) return;
+   const u64 b0 = ibyte[i] * 8;
+   put_bits_or(outw, b0, 0x425A6830u + level, 32);
+   u32 c = 0;
+   u64 end = b0 + 32;
+   for (u32 b = first[i]; b < first[i + 1]; b++) { c = ((c << 1) | (c >> 31)) ^ crc[b]; end += bits[b]; }
+   put_bits_or(outw, end, 0x177245385090ULL, 48);
+   put_bits_or(outw, end + 48, c, 32);
+   icrc[i] = c;
+}
+
+static int stage4_frames(Engine* e, u32 n_items, u32 nb, u8* d_out)
+{
+   cudaStream_t st = e->stream;
+   k_item_frames<<<(n_items + 255) / 256, 256, 0, st>>>(reinterpret_cast<u32*>(d_out), e->it.byteoff, e->bt.bits,
+                                                         e->it.first, e->bt.crc, e->it.crc, n_items, (u32)e->level); BZ_KCHECK(e);
+   BZ_CUDA(e, cudaMemcpyAsync(e->h_scalars + 16, e->bt.bitoff + nb, sizeof(u64), cudaMemcpyDeviceToHost, st));
+   BZ_CUDA(e, cudaStreamSynchronize(st));
+   return 0;
+}
+
+// a batch window whose items are all empty: headers and trailers only
+int stage4_empty_items(Engine* e, u32 n_items, u8* d_out, u64* end_bit_out)
+{
+   k_item_offsets<<<1, 1024, 0, e->stream>>>(e->bt.bits, e->bt.bitoff, e->it.first, n_items, e->it.byteoff); BZ_KCHECK(e);
+   const int rc = stage4_frames(e, n_items, 0, d_out);
+   if (rc) return rc;
+   *end_bit_out = *reinterpret_cast<u64*>(e->h_scalars + 16);
+   return 0;
+}
+
 int put_bits_device(Engine* e, u8* d_out, u64 origin_bit, u64 bitpos, u64 value, int nbits)
 {
    k_put_bits<<<1, 1, 0, e->stream>>>(reinterpret_cast<u32*>(d_out), bitpos - origin_bit, value, nbits);
@@ -552,7 +641,7 @@ int put_bits_device(Engine* e, u8* d_out, u64 origin_bit, u64 bitpos, u64 value,
    return 0;
 }
 
-int stage4_run(Engine* e, u32 nb, u32 E, u8* d_out, u64 origin_bit, u64 start_bit, u64* end_bit_out)
+int stage4_run(Engine* e, u32 nb, u32 E, u8* d_out, u64 origin_bit, u64 start_bit, u64* end_bit_out, u32 n_items)
 {
    (void)E;
    cudaStream_t st = e->stream;
@@ -573,12 +662,19 @@ int stage4_run(Engine* e, u32 nb, u32 E, u8* d_out, u64 origin_bit, u64 start_bi
    }
    BZ_CUDA(e, cudaMemsetAsync(e->pre, 0, (size_t)PRE_STRIDE * nb, st));
    k_huff_finish<<<nb, 192, 0, st>>>(p);                                                     BZ_KCHECK(e);
-   k_bit_offsets<<<1, 1024, 0, st>>>(e->bt.bits, e->bt.bitoff, nb, start_bit);               BZ_KCHECK(e);
+   if (n_items) { k_item_offsets<<<1, 1024, 0, st>>>(e->bt.bits, e->bt.bitoff, e->it.first, n_items, e->it.byteoff); BZ_KCHECK(e); }
+   else { k_bit_offsets<<<1, 1024, 0, st>>>(e->bt.bits, e->bt.bitoff, nb, start_bit);        BZ_KCHECK(e); }
    k_huff_select<1><<<gsel, SEL_THREADS, 0, st>>>(p);                                        BZ_KCHECK(e);
    k_group_scan<<<nb, 1024, 0, st>>>(p);                                                     BZ_KCHECK(e);
    u32* outw = reinterpret_cast<u32*>(d_out);
    k_pack<<<gsel, SEL_THREADS, 0, st>>>(p, outw, origin_bit);                                BZ_KCHECK(e);
    k_pre_copy<<<dim3((PRE_STRIDE / 4 + 255) / 256, nb), 256, 0, st>>>(p, outw, origin_bit);  BZ_KCHECK(e);
+   if (n_items) {
+      const int rc = stage4_frames(e, n_items, nb, d_out);
+      if (rc) return rc;
+      *end_bit_out = *reinterpret_cast<u64*>(e->h_scalars + 16);
+      return 0;
+   }
    BZ_CUDA(e, cudaMemcpyAsync(e->h_scalars + 16, e->bt.bitoff + nb, sizeof(u64), cudaMemcpyDeviceToHost, st));
    BZ_CUDA(e, cudaStreamSynchronize(st));
    *end_bit_out = *reinterpret_cast<u64*>(e->h_scalars + 16);

@@ -13,6 +13,7 @@
  *                                      BZ2_compressBlock per block (compress.c:822-881),
  *                                      i.e. the body of BZ2_bzBuffToBuffCompress (bzlib.c:1309-1357)
  *   bz2b200_compress_device            same, input and output resident in HBM
+ *   bz2b200_compress_batch_*           the same for many inputs at once, one stream each
  *   bz2b200_stream_*                   the same work fed in pieces (BZ2_bzCompress with
  *                                      BZ_RUN / BZ_FLUSH / BZ_FINISH, bzlib.c:400-454)
  *   bz2b200_debug_*                    per-stage intermediates for parity tests (the
@@ -93,6 +94,33 @@ int  bz2b200_compress_host(bz2b200_engine* e, const void* src, size_t src_len,
 int  bz2b200_compress_device(bz2b200_engine* e, const void* d_src, size_t src_len,
                              void* d_dst, size_t dst_cap, size_t* dst_len, unsigned flags,
                              bz2b200_stats* stats);
+
+/* ---- many independent inputs in one call ---------------------------------------------------------
+ * Consecutive items are packed into windows; no run, chunk or block crosses from one item into the next, and each
+ * item is framed as its own stream.  An item too large for one window goes through the single-stream window loop. */
+
+/* Worst-case size of one stream: the reference's documented BuffToBuff bound (1% + 600 bytes). */
+size_t bz2b200_compress_bound(int block_size_100k, size_t n);
+
+/* An engine whose windows can hold up to max_items inputs of a batch (block slots = full blocks of a window +
+ * max_items, at most 4096).  Each extra slot costs about hist_stride*4 + 280*nmax/1024 + 25 KB of HBM (~1.3 MB at -9). */
+int  bz2b200_engine_create_batch(bz2b200_engine** out, int device, int block_size_100k, size_t window_bytes, size_t max_items);
+
+/* Item k is src[offs[k], offs[k+1]) (offs: host array of n_items+1, non-decreasing, offs[0] = 0).  Each item becomes its
+ * own complete .bz2 stream, byte-identical to bz2b200_compress_host(e, item, flags) on that item alone.  The streams are
+ * written back to back: stream k is dst[out_offs[k], out_offs[k+1]), so dst[0, out_offs[n]) is a valid multi-stream
+ * .bz2 file and out_offs is its index.  stream_crcs (optional, n_items) receives each stream's combined CRC.
+ * flags: 0 or BZ2B200_TAIL_STREAMED, applied to every item; NO_HEADER / NO_TRAILER are EPARAM.
+ * dst too small: BZ2B200_EOUTFULL, and nothing is written past dst_cap.  Any engine but a bounded one accepts a batch;
+ * one from bz2b200_engine_create_batch packs more items per window.  Stats are summed over the call; combined_crc is 0
+ * and out_bits is 8 x the bytes written. */
+int  bz2b200_compress_batch_host(bz2b200_engine* e, const void* src, const uint64_t* offs, size_t n_items,
+                                 void* dst, size_t dst_cap, uint64_t* out_offs, uint32_t* stream_crcs,
+                                 unsigned flags, bz2b200_stats* stats);
+/* The same with src and dst in device memory (offs, out_offs and stream_crcs stay host arrays; no alignment needed). */
+int  bz2b200_compress_batch_device(bz2b200_engine* e, const void* d_src, const uint64_t* offs, size_t n_items,
+                                   void* d_dst, size_t dst_cap, uint64_t* out_offs, uint32_t* stream_crcs,
+                                   unsigned flags, bz2b200_stats* stats);
 
 /* Streaming: feed input in pieces; compressed bytes are handed to `sink`.
  * end_mode: 0 = more input will follow (BZ_RUN), 1 = flush (BZ_FLUSH: close the open
